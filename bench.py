@@ -2,10 +2,11 @@
 """bench.py - Groth16 proofs/sec (BN254, 2^20-constraint-domain circom squaring chain) on B200, next to the CPU path.
 
 One "step" = one call of Groth16::<Bn254, CircomReduction>::create_proof_with_reduction_and_matrices
-(/root/reference/benches/groth16.rs:69-84 times exactly this): proving key + matrices resident, witness given, fixed r, s.
+(ark-circom's benches/groth16.rs:69-84 times exactly this): proving key + matrices resident, witness given, fixed r, s.
 
   python bench.py [--gpus N --steps K --warmup W]        our arm (CUDA, through the C ABI)
   python bench.py --impl reference [...]                 the CPU restatement of the ark-groth16 0.5 path (oracle/cref.c)
+  python bench.py [...] --dump-outputs DIR               also write the proof of the last timed step to DIR (dump_outputs)
 
 Output: ONE JSON line (rank 0).  `value` = device-resident throughput (witness already in HBM), `e2e` = through
 Groth16.create_proof_with_reduction_and_matrices with a pinned HOST witness (H2D 32 B x n_vars and D2H 256 B inside the
@@ -24,6 +25,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 R_FIX = 0x1234567890abcdef1234567890abcdef
 S_FIX = 0xfedcba0987654321fedcba0987654321
@@ -163,6 +165,20 @@ def workload_config(args, circ):
             "l2": "inputs larger than L2 (proving-key tables ~6 GB per proof pass vs 126 MB L2)"}
 
 
+def dump_outputs(out_dir, proof_bytes):
+    """What the caller of the timed path receives from its last step: the 256-byte Proof (canonical little-endian affine
+    coordinates), written as proof_a.npy (2, 32), proof_b.npy (2, 2, 32) and proof_c.npy (2, 32) in the order of Proof.a /
+    Proof.b / Proof.c.  One float32 per byte: every value is exact, and a one-bit difference moves a value by at least 1.
+    The inputs (synthetic key seed, witness, r, s) are fixed, so two builds given the same arguments must write the same files."""
+    import numpy as np
+    b = np.frombuffer(proof_bytes, dtype=np.uint8).astype(np.float32)
+    assert b.size == 256, b.size
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (('proof_a', b[:64].reshape(2, 32)), ('proof_b', b[64:192].reshape(2, 2, 32)), ('proof_c', b[192:].reshape(2, 32))):
+        np.save(os.path.join(out_dir, name + '.npy'), arr)
+    log(f"[bench] last timed proof written to {out_dir}/proof_{{a,b,c}}.npy")
+
+
 def run_reference(args):
     rank = int(os.environ.get('RANK', '0'))
     if rank != 0:
@@ -185,9 +201,11 @@ def run_reference(args):
     t0 = time.perf_counter()
     for _ in range(args.steps):
         t1 = time.perf_counter()
-        cref.prove(za, R_FIX, S_FIX, wm, nthreads=cores)
+        proof = cref.prove(za, R_FIX, S_FIX, wm, nthreads=cores)
         steps.append(time.perf_counter() - t1)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof)
     val = args.steps / dt
     sample = f"{args.steps} full proofs of the {args.workload} 2^{args.log_n} workload, oracle/cref.c (C + OpenMP restatement of ark-groth16 0.5), {cores} threads pinned one per core"
     out = {"impl": "reference", "metric": METRIC, "value": val, "unit": "proofs/s", "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -409,8 +427,10 @@ def run_ours(args):
     wl = Workload(args.log_n, args.workload, inflight)
     main_mode = 'single' if world == 1 else args.mode
     main = measure(wl, main_mode, args.steps, args.warmup, inflight)
-    proof = main["proof"]
+    proof = main["proof"]                                                 # the last step of the timed e2e loop
     ctx = main["ctxs"][0]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof.data)
 
     if rank == 0 and not args.skip_check:
         wl.check_closed_form(proof)
@@ -555,11 +575,14 @@ def main():
     ap.add_argument('--host-driver', default='async', choices=['async', 'threads'], help="e2e loop: one host thread with b2g_prove_submit/wait (async) or one thread per in-flight proof")
     ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
     ap.add_argument('--skip-check', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the proof of the last timed step as DIR/proof_{a,b,c}.npy')
     args = ap.parse_args()
     if args.steps is None:
         args.steps = 3 if args.impl == 'reference' else 20
     if args.warmup is None:
         args.warmup = 1 if args.impl == 'reference' else 3
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be at least 1 and --warmup at least 0')
     if args.impl == 'reference':
         run_reference(args)
     else:

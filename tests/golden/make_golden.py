@@ -1,8 +1,8 @@
-"""Generates tests/golden/golden_vectors.json.  Run in the build container (needs /root/reference):
-    python tests/golden/make_golden.py
-Sources of every value:
+"""Generates tests/golden/golden_vectors.json from a checkout of the reference, ark-circom (arkworks-rs/circom-compat):
+    python tests/golden/make_golden.py <path to the ark-circom checkout>
+The tests only read the JSON this writes; they never need the checkout.  Sources of every value:
   * kat_fq_one / kat_g1_one / kat_g2_one : byte vectors printed by snarkjs and pinned by the reference's own tests
-    (/root/reference/src/zkey.rs:398-432, expectations :435-463) - extracted from that file by regex, not retyped.
+    (src/zkey.rs:398-432, expectations :435-463) - extracted from that file by regex, not retyped.
   * test_zkey / complex_zkey proofs: computed by oracle/pyref.py (big-int arithmetic, independent of the C and CUDA
     code) for fixed (r, s); each proof is checked with the pairing verifier before it is written.  They equal the
     self-derived vectors of SURVEY.md App. E.
@@ -18,7 +18,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, '..', '..'))
 from oracle import pyref as o  # noqa: E402
 
-REF = '/root/reference'
+REF = None                                               # the ark-circom checkout, from the command line
 R = 0x1234567890abcdef1234567890abcdef
 S = 0xfedcba0987654321fedcba0987654321
 
@@ -29,7 +29,7 @@ def rust_byte_vec(src, fn_name):
 
 
 def deser_key_kat(src):
-    """The reference's largest known-answer test, `fn deser_key` (/root/reference/src/zkey.rs:545-763): every point of
+    """The reference's largest known-answer test, `fn deser_key` (src/zkey.rs:545-763): every point of
     test.zkey's IC / A / B1 / B2 / L / H queries as the raw bytes it feeds to deserialize_g1 / deserialize_g2.  Extracted
     by regex from that function's body (not retyped): {field: [[byte, ...] per point]}."""
     body = re.search(r'fn deser_key\(\) \{(.*?)\n    \}\n', src, re.S).group(1)
@@ -113,4 +113,7 @@ def main():
 
 
 if __name__ == '__main__':
+    if len(sys.argv) != 2 or not os.path.isfile(os.path.join(sys.argv[1], 'src', 'zkey.rs')):
+        sys.exit('usage: python tests/golden/make_golden.py <path to the ark-circom checkout>')
+    REF = sys.argv[1]
     main()
