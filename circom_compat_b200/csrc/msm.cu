@@ -82,6 +82,7 @@ __device__ __forceinline__ int32_t msm_digit_at(const uint32_t* __restrict__ k, 
         if (b < half - 1) break;
     }
     const uint32_t coef = msm_window_bits(k, c, w) + carry;
+    // top window: k < r keeps coef < 2^(c-1) for c in [8, 22], so cout = 0 and dropping it loses nothing (test_msm_digit_model.py)
     const uint32_t cout = (coef + half) >> c;
     return (int32_t)coef - (int32_t)(cout << c);
 }
